@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — admission decisions/sec of the batched scheduling-cycle evaluator.
 
-    python bench.py --gpus N --steps K --warmup W [--config 2] [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--config 2] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one scheduling cycle (tree pass -> nominate [+ target search] -> group ->
 order -> admit) over one synthetic snapshot of a BASELINE.json configuration.  Default
@@ -17,6 +17,10 @@ independent, so there is no data-path collective) — weak scaling.
 
 --impl reference times the CPU restatement of the reference's cycle (oracle/, the
 Go toolchain is absent so the Go scheduler itself cannot run here) on the host cores.
+
+--dump-outputs DIR writes the tables the last timed step handed its caller (rank 0's) as
+DIR/<name>.npy; tables without rows are left out.  Inputs are seeded, so two builds, or the two --impl arms, run with the same
+arguments can be compared table by table.
 """
 from __future__ import annotations
 
@@ -47,6 +51,42 @@ WORKLOADS = {
 # cfg3 runs the fair-sharing iterator, which holds one entry per ClusterQueue
 # (fair_sharing_iterator.go:52-54): its step is one reference cycle over the Q heads.
 HEADS = {1: "all", 2: "all", 3: "one_per_cq", 4: "one_per_cq", 5: "one_per_cq"}
+DUMP_LIMIT = 64 << 20
+
+
+def cycle_tables(out) -> dict:
+    """The result tables of one scheduling cycle (abi.CycleOut), target lists cut to their used length."""
+    t = {f: getattr(out, f) for f in ("decision", "mode", "borrow", "commit_rank", "ps_flavor", "ps_res_mode", "ps_tried_idx",
+                                      "ps_count", "tgt_start", "node_usage")}
+    t["tgt_adm"], t["tgt_reason"] = out.tgt_adm[:out.n_targets], out.tgt_reason[:out.n_targets]
+    return t
+
+
+def tas_tables(out, n_req: int) -> dict:
+    """The result tables of one kb_tas_find (tas.TasOut), cut to the requests and assignments actually written."""
+    n = int(out.asg_start[-1])
+    return {"status": out.status[:n_req], "asg_start": out.asg_start, "asg_leaf": out.asg_leaf[:n], "asg_count": out.asg_count[:n]}
+
+
+def dump_outputs(path: str, tables: dict) -> None:
+    """Writes every table as <path>/<name>.npy: integers of up to 16 bits as float32, wider ones as float64 (exact up
+    to 2^53, checked).  A table without rows is left out: the target lists of a cycle that preempts nothing are
+    empty, and tgt_start already says so."""
+    conv = {}
+    for name, a in tables.items():
+        a = np.asarray(a)
+        if a.size == 0:
+            continue
+        f = a.astype(np.float32 if a.dtype.itemsize <= 2 else np.float64)
+        if not np.array_equal(f.astype(a.dtype), a):
+            raise ValueError(f"--dump-outputs: {name} is not exact in {f.dtype}")
+        conv[name] = f
+    total = sum(f.nbytes for f in conv.values())
+    if total > DUMP_LIMIT:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(path, exist_ok=True)
+    for name, f in conv.items():
+        np.save(os.path.join(path, name + ".npy"), f)
 
 
 def algorithmic_bytes(snap) -> dict:
@@ -237,11 +277,13 @@ def run_tas(args, rank, world, local_rank):
     dev_ms, kms, launches = 0.0, np.zeros(20), 0
     for _ in range(args.steps):
         flush.zero_(); torch.cuda.synchronize()
-        ev.tas_find(topo, reqs, cap)
+        last = ev.tas_find(topo, reqs, cap)
         st = ev.stats()
         dev_ms += st.last_cycle_gpu_ms; kms += np.array(list(st.kernel_ms)); launches += st.kernel_launches
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, tas_tables(last, nreq))
     t0 = time.perf_counter()
     for _ in range(args.steps):
         out = ev.tas_find(topo, reqs, cap)
@@ -316,8 +358,10 @@ def run_reference(args, rank, world):
             oracle.tas_find(topo, sample)
         t0 = time.perf_counter()
         for _ in range(args.steps):
-            oracle.tas_find(topo, sample)
+            last = oracle.tas_find(topo, sample)
         dt = time.perf_counter() - t0
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, tas_tables(last, 400))
         val = args.steps * 400 / dt
         print(json.dumps({"impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
                           "ms_per_step": dt / args.steps * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "int64", "data": "synthetic",
@@ -332,8 +376,10 @@ def run_reference(args, rank, world):
         oracle.run_cycle(snap)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        oracle.run_cycle(snap)
+        last = oracle.run_cycle(snap)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, cycle_tables(last))
     val = args.steps * snap.n_heads / dt
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": dt / args.steps * 1e3, "higher_is_better": True, "scaling": "weak",
@@ -364,7 +410,12 @@ def main():
     ap.add_argument("--l2", default="rotate", choices=["rotate", "flush"],
                     help="how inputs are kept out of L2 between timed steps: rotate = device-resident copies of the snapshot "
                          "whose total exceeds L2, used round-robin; flush = a 512 MiB buffer is written before every step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the tables the last timed step returned (rank 0's) as DIR/<name>.npy, "
+                         f"float32 / float64, at most {DUMP_LIMIT >> 20} MiB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
@@ -459,6 +510,10 @@ def main():
     barrier()
     wall_ms = (time.perf_counter() - t_wall0) * 1e3
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        # the tables of the last timed step, as kb_download hands them to a caller of the resident path
+        last = evs[(args.steps - 1) % len(evs)].download(snap, abi.CycleOut(snap))
+        dump_outputs(args.dump_outputs, cycle_tables(last))
     # per-kernel split (roofline.kernel_ms): the same K steps once more with an event before every kernel; not part of
     # `value` (the extra event records sit between the kernels of the timed stream)
     _, _, kms = timed_pass(args.steps, use_flush, True)

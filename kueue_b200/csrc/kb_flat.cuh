@@ -5,9 +5,11 @@
 // one idea: the CTA first RELOCATES its root's slice of the snapshot into shared memory — quota tables, the static
 // per-ClusterQueue policy / resource-group tables (one contiguous host-built block per tree, DevSnap::tree_blob) and
 // the per-cycle head / podset records of its entries — renumbering every id (entry, workload, podset row,
-// ClusterQueue, resource group) to be local to the root.  The flavor assigner, the iterator key and the request
-// expansion are the SAME device functions every other kernel uses (assign_workload_coop, compute_entry_key,
-// expand_entry): they run on a DevSnap whose table pointers all point into that relocated copy (tab_local == 2), so
+// ClusterQueue, resource group) to be local to the root.  Heads with one podset and no PodSetReducer take a flavor
+// walk, DRS term and request row specialised to the flat tree (flat_walk, flat_share_ratio).  For every other head the
+// flavor assigner, the DRS term and the request expansion are the SAME device functions every other kernel uses
+// (get_assignments_coop, entry_share_ratio, expand_entry): they run on a DevSnap whose table pointers all point into
+// that relocated copy (tab_local == 2), so
 // their chains of dependent loads (head -> workload -> podset rows -> resource group -> flavors -> quota cells) cost
 // shared-memory latency instead of an L2 / HBM round trip per hop.  Global memory is touched in two bursts: the
 // staging at the start (every load independent, at most three dependent hops: tree_start -> node / head record ->
@@ -19,7 +21,7 @@
 
 struct FlatLay {  // byte offsets into the dynamic shared memory of k_cycle_flat (computed on the host, passed by value)
   uint32_t u, sub, lq, bl, av, pot, over, lend, blob, n_e, n_wl, n_ps0, n_psn, e_gid, e_cq, e_prio, e_ident, e_psn, e_wl, e_ps0, e_ts, e_lg, e_qr,
-      e_mode, e_borrow, e_rank, sorted, m_sorted, d_sorted, r_gid, r_count, r_min, r_mask, r_group, r_ok, r_req, r_last, o_fl, o_md, o_tr, o_cnt, key, misc, snap, rec, total;
+      e_flat, e_mode, e_borrow, e_rank, sorted, m_sorted, d_sorted, r_gid, r_count, r_min, r_mask, r_group, r_ok, r_req, r_last, o_fl, o_md, o_tr, o_cnt, key, misc, snap, rec, total;
 };
 __host__ __device__ inline FlatLay flat_layout(int ncap, int FR, int R, int rcap, int bcap) {
   FlatLay L;
@@ -32,7 +34,7 @@ __host__ __device__ inline FlatLay flat_layout(int ncap, int FR, int R, int rcap
   L.n_e = take((size_t)ncap * 4); L.n_wl = take((size_t)ncap * 4); L.n_ps0 = take((size_t)ncap * 4); L.n_psn = take((size_t)ncap * 4);
   L.e_gid = take((size_t)ncap * 4); L.e_cq = take((size_t)ncap * 4); L.e_prio = take((size_t)ncap * 4); L.e_ident = take((size_t)ncap * 4);
   L.e_psn = take((size_t)(ncap + 1) * 4); L.e_wl = take((size_t)ncap * 4); L.e_ps0 = take((size_t)ncap * 4);
-  L.e_ts = take((size_t)ncap * 8); L.e_lg = take((size_t)ncap * 8); L.e_qr = take((size_t)ncap);
+  L.e_ts = take((size_t)ncap * 8); L.e_lg = take((size_t)ncap * 8); L.e_qr = take((size_t)ncap); L.e_flat = take((size_t)ncap);
   L.e_mode = take((size_t)ncap * 4); L.e_borrow = take((size_t)ncap * 4); L.e_rank = take((size_t)ncap * 4);
   L.sorted = take((size_t)ncap * 4); L.m_sorted = take((size_t)ncap * 4); L.d_sorted = take(((size_t)ncap / 32 + 2) * 4);
   L.r_gid = take((size_t)rcap * 4); L.r_count = take((size_t)rcap * 4); L.r_min = take((size_t)rcap * 4); L.r_mask = take((size_t)rcap * 4);
@@ -181,6 +183,202 @@ __device__ __forceinline__ int flat_decision(int mode, const uint32_t *ok_bits, 
   return mode == KB_MODE_PREEMPT ? KB_DEC_PREEMPT_NO_TARGETS : KB_DEC_NOFIT;
 }
 
+// e_flat bits of an entry, set when its records are gathered
+enum {
+  KB_FLAT_WALK = 1,  // one podset and no PodSetReducer (not: PartialAdmission, min_count >= 0, count > min_count)
+  KB_FLAT_PODS = 2   // its ClusterQueue has a resource group with the pods resource (covers_pods)
+};
+
+// get_assignments_coop for an entry with KB_FLAT_WALK, on the relocated tables.  With one podset there is no usage
+// assumed from earlier podsets, no PodSetGroup and no count scaling: request(r) = ps_req, or the pod count for the pods
+// resource (ps_request).  On a flat tree every ClusterQueue's parent is the root, which has no parent, so find_height
+// is closed form: over nominal (usage + val > nominal) -> height of the root and no reclaim, else 0 and may reclaim.
+// No ClusterQueue of a relocated root has preemption candidates, so the oracle's answer is always PM_NOCAND.
+// Tables are addressed from the layout (shared-memory offsets), not through the relocated DevSnap.  Same results
+// (rows, mode, borrowing) as get_assignments_coop; lane 0 of the group writes them.
+template <int NG>
+__device__ __forceinline__ void flat_walk(const DevSnap &D, const FlatLay &Y, unsigned char *sm, int i, unsigned gmask, int gbase, int glane) {
+  const int R = D.R, FR = D.FR;
+  const unsigned char *blob = sm + Y.blob;
+  const TreeBlobHdr &BH = *(const TreeBlobHdr *)blob;
+  const i64 *s_u = (const i64 *)(sm + Y.u), *s_sub = (const i64 *)(sm + Y.sub), *s_av = (const i64 *)(sm + Y.av), *s_pot = (const i64 *)(sm + Y.pot);
+  const int cq = ((const int *)(sm + Y.e_cq))[i], l = ((const int *)(sm + Y.e_psn))[i];
+  const bool covers_pods = sm[Y.e_flat + i] & KB_FLAT_PODS;
+  const int full = ((const int *)(sm + Y.r_count))[l];
+  const uint32_t mask = ((const uint32_t *)(sm + Y.r_mask))[l] | (covers_pods ? 1u << D.pods_res : 0u);
+  const u64 ok = ((const u64 *)(sm + Y.r_ok))[l];
+  const i64 *req = (const i64 *)(sm + Y.r_req) + (size_t)l * R;
+  const i64 lg = ((const i64 *)(sm + Y.e_lg))[i];
+  const bool use_last = lg >= 0 && !(((const i64 *)(blob + BH.gen))[cq] > lg);
+  const bool fung = D.flags & KB_F_FLAVOR_FUNGIBILITY;
+  const int pref = blob[BH.pref + cq], wcb = blob[BH.wcb + cq], wcp = blob[BH.wcp + cq];
+  const bool can_pwb = blob[BH.borrow_w + cq] != KB_POLICY_NEVER || ((D.flags & KB_F_FAIR_SHARING) && blob[BH.reclaim + cq] != KB_POLICY_NEVER);
+  const int h_root = ((const int32_t *)(blob + BH.hgt))[0];
+  const int32_t *rg_start = (const int32_t *)(blob + BH.rgs), *rg_fl = (const int32_t *)(blob + BH.rgfl), *fls = (const int32_t *)(blob + BH.fl);
+  const uint32_t *rg_mask = (const uint32_t *)(blob + BH.rgmask);
+  const int g0 = rg_start[cq], g1 = rg_start[cq + 1];
+  int8_t *o_fl = (int8_t *)(sm + Y.o_fl) + (size_t)l * R, *o_md = (int8_t *)(sm + Y.o_md) + (size_t)l * R, *o_tr = (int8_t *)(sm + Y.o_tr) + (size_t)l * R;
+  auto request = [&](int r) { return covers_pods && r == D.pods_res ? (i64)full : req[r]; };
+  if (glane == 0) {
+    for (int r = 0; r < R; r++) { o_fl[r] = -1; o_md[r] = -1; o_tr[r] = -1; }
+    ((int *)(sm + Y.o_cnt))[l] = full;
+  }
+  bool has_reasons = false, failed = false;
+  int ps_borrow = 0;
+  uint32_t assigned = 0, ps_pmask = 0;
+  for (int r0 = 0; r0 < R; r0++) {
+    if (!(mask & (1u << r0)) || (assigned & (1u << r0))) continue;
+    int g = -1;
+    for (int k = g0; k < g1 && g < 0; k++) if (rg_mask[k] & (1u << r0)) g = k;
+    if (g < 0) {
+      if (request(r0) == 0) continue;
+      failed = true; break;
+    }
+    const uint32_t rgm = rg_mask[g] & mask;
+    const int fl0 = rg_fl[g], nfl = rg_fl[g + 1] - fl0;
+    int best_f = -1, best_pm = PM_NOFIT, best_rb = INT32_MAX, best_maxb = 0;
+    uint32_t best_pmask = 0;
+    bool any_reason = false, done = false;
+    int attempted = -1;
+    const int idx0 = fung && use_last ? ((const int8_t *)(sm + Y.r_last))[(size_t)l * R + r0] + 1 : 0;
+    for (int base = idx0; base < nfl && !done; base += NG) {
+      // ---- one flavor per lane: every cell of the group is loaded before the first is decided ----
+      const int idx = base + glane;
+      u64 res = 0;  // packed as in assign_workload_coop
+      int myf = -1;
+      if (idx < nfl) {
+        const int f = fls[fl0 + idx];
+        myf = f;
+        if ((ok >> f) & 1) {
+          int rpm = PM_FIT, rb = 0, maxb = 0; uint32_t pmask = 0; bool reason = false;
+          for (int rc = 0; rc < R && rpm != PM_NOFIT; rc += 4) {
+            int pmv[4], bv[4];
+#pragma unroll
+            for (int j = 0; j < 4; j++) {  // cell_eval
+              const int r = rc + j;
+              pmv[j] = PM_FIT; bv[j] = 0;
+              if (r < R && (rgm & (1u << r))) {
+                const int c = cq * FR + f * R + r;
+                const i64 val = request(r), pot = s_pot[c], nom = s_sub[c], u = s_u[c], av = s_av[c];
+                const bool over = u + val > nom;
+                if (val > pot) pmv[j] = PM_NOFIT;
+                else {
+                  bv[j] = over ? h_root : 0;
+                  if (!(val <= imax(0, av))) pmv[j] = (val <= nom || !over || can_pwb) ? PM_NOCAND : PM_NOFIT;
+                }
+              }
+            }
+#pragma unroll
+            for (int j = 0; j < 4; j++) {
+              const int r = rc + j;
+              if (r >= R || !(rgm & (1u << r))) continue;
+              const int pm = pmv[j], b = bv[j];
+              if (pm != PM_FIT) reason = true;
+              if (gm_preferred(rpm, rb, pm, b, pref)) { rpm = pm; rb = b; }
+              if (rpm == PM_NOFIT) break;
+              if (fa_mode(pm) == KB_MODE_PREEMPT) pmask |= 1u << r;
+              if (b > maxb) maxb = b;
+            }
+          }
+          res = (u64)rpm | ((u64)(rb & 127) << 3) | ((u64)(maxb & 127) << 10) | ((u64)reason << 17) | (1ull << 19) | ((u64)pmask << 32);
+        }
+      }
+      // ---- ordered scan over the flavors of this round (assign_workload_coop) ----
+      for (int j = 0; j < NG && base + j < nfl; j++) {
+        const u64 rj = __shfl_sync(gmask, res, gbase + j);
+        const int fj = __shfl_sync(gmask, myf, gbase + j);
+        attempted = base + j;
+        if (!((rj >> 19) & 1)) { any_reason = true; continue; }
+        const int rpm = (int)(rj & 7), rb = (int)((rj >> 3) & 127), maxb = (int)((rj >> 10) & 127);
+        const uint32_t pmask = (uint32_t)(rj >> 32) & 0xffffu;
+        if ((rj >> 17) & 1) any_reason = true;
+        bool take = false;
+        if (fung) {
+          const bool try_next = rpm == PM_NOFIT || rpm == PM_NOCAND ||
+                                ((rpm == PM_PREEMPT || rpm == PM_RECLAIM) && wcp == KB_FUNG_TRY_NEXT_FLAVOR) ||
+                                (rb != 0 && wcb == KB_FUNG_TRY_NEXT_FLAVOR);
+          if (!try_next) { take = true; done = true; }
+          else if (gm_preferred(rpm, rb, best_pm, best_rb, pref)) take = true;
+        } else if (rpm > best_pm) {
+          take = true;
+          done = rpm == PM_FIT;
+        }
+        if (take) { best_f = fj; best_pm = rpm; best_rb = rb; best_maxb = maxb; best_pmask = pmask; }
+        if (done) break;
+      }
+    }
+    if (best_f < 0) { failed = true; break; }
+    const int tried = fung ? (attempted == nfl - 1 ? -1 : attempted) : 0;
+    if (glane == 0)
+      for (int r = 0; r < R; r++) {
+        if (!(rgm & (1u << r))) continue;
+        o_fl[r] = (int8_t)best_f; o_md[r] = (best_pmask >> r) & 1 ? KB_MODE_PREEMPT : KB_MODE_FIT; o_tr[r] = (int8_t)tried;
+      }
+    assigned |= rgm;
+    ps_pmask |= best_pmask & rgm;
+    if (best_maxb > ps_borrow) ps_borrow = best_maxb;
+    if (best_pm != PM_FIT && any_reason) has_reasons = true;
+  }
+  int mode = KB_MODE_FIT, borrowing = ps_borrow;
+  if (failed) {
+    mode = KB_MODE_NOFIT; borrowing = 0;
+    if (glane == 0) for (int r = 0; r < R; r++) { o_fl[r] = -1; o_md[r] = -1; o_tr[r] = -1; }
+  } else if (has_reasons) {
+    if ((assigned & mask) == 0) mode = KB_MODE_NOFIT;
+    else if (ps_pmask & mask) mode = KB_MODE_PREEMPT;
+  }
+  if (glane == 0) { ((int *)(sm + Y.e_mode))[i] = mode; ((int *)(sm + Y.e_borrow))[i] = borrowing; }
+}
+
+// entry_share_ratio of a KB_FLAT_WALK entry: its one podset puts request(r) on a single cell (flavor o_fl[r]), counted
+// at its full count, and the ClusterQueue's parent is the root (local handle 0)
+__device__ __forceinline__ double flat_share_ratio(const DevSnap &D, const FlatLay &Y, const unsigned char *sm, int i, int r) {
+  const int R = D.R;
+  const int hq = ((const int *)(sm + Y.e_cq))[i], l = ((const int *)(sm + Y.e_psn))[i];
+  i64 b = ((const i64 *)(sm + Y.over))[hq * R + r];
+  const int f = ((const int8_t *)(sm + Y.o_fl))[(size_t)l * R + r];
+  if (f >= 0) {
+    const i64 q = (sm[Y.e_flat + i] & KB_FLAT_PODS) && r == D.pods_res ? (i64)((const int *)(sm + Y.o_cnt))[l] : ((const i64 *)(sm + Y.r_req))[(size_t)l * R + r];
+    const int c = hq * D.FR + f * R + r;
+    const i64 base = ((const i64 *)(sm + Y.u))[c] - ((const i64 *)(sm + Y.sub))[c];
+    b += imax(0, base + (q > 0 ? q : 0)) - imax(0, base);
+  }
+  const i64 lend = ((const i64 *)(sm + Y.lend))[r];
+  return (b > 0 && lend > 0) ? (double)b * 1000.0 / (double)lend : 0.0;
+}
+// entry_key_finish on the relocated records (local workload = local entry); the key reads no podset
+__device__ __forceinline__ void flat_key_finish(const DevSnap &D, const FlatLay &Y, const unsigned char *sm, int i, bool fair, double best, u64 *k) {
+  unsigned prio = 0;
+  if (D.flags & KB_F_PRIORITY_SORTING_WITHIN_COHORT) prio = ~((unsigned)((const int *)(sm + Y.e_prio))[i] ^ 0x80000000u);
+  const u64 ts = (u64)((const i64 *)(sm + Y.e_ts))[i] ^ 0x8000000000000000ull;
+  const int borrow = ((const int *)(sm + Y.e_borrow))[i];
+  if (!fair) {
+    const u64 no_qr = (D.wl_has_qr && sm[Y.e_qr + i]) ? 0ull : 1ull;
+    k[0] = (no_qr << 63) | ((u64)(unsigned)borrow << 32) | prio; k[1] = ts; k[2] = (u64)(unsigned)((const int *)(sm + Y.e_gid))[i]; k[3] = 0;
+    return;
+  }
+  const unsigned char *blob = sm + Y.blob;
+  const TreeBlobHdr &BH = *(const TreeBlobHdr *)blob;
+  const int cq = ((const int *)(sm + Y.e_cq))[i];
+  const double w = ((const double *)(blob + BH.wgt))[cq];
+  const bool zwb = w == 0 && best != 0;
+  const double value = zwb ? best : (best == 0 ? 0.0 : best / w);
+  const u64 vb = (u64)__double_as_longlong(value);
+  const u64 flags = ((D.flags & KB_F_FS_PRIORITIZE_NON_BORROWING) && borrow > 0 ? 2 : 0) | (zwb ? 1 : 0);
+  k[0] = (flags << 32) | (vb >> 32); k[1] = (vb << 32) | prio; k[2] = ts; k[3] = (u64)(unsigned)((const int32_t *)(blob + BH.gid))[cq];
+}
+
+// get_assignments_coop for the entries without KB_FLAT_WALK, kept out of line: its inlined copies of
+// assign_workload_coop (four, three of them for the PodSetReducer) would otherwise share the kernel's 64 registers
+// with the rest of the cycle and push its long-lived values to the stack.
+template <int NG>
+__device__ __noinline__ void flat_generic_assign(const DevSnap &L, int i, unsigned gmask, int gbase, int glane, int *e_mode, int *e_borrow) {
+  bool need_search = false;
+  int borrowing;
+  const int mode = get_assignments_coop<NG>(L, &need_search, i, &borrowing, gmask, gbase, glane);
+  if (glane == 0) { e_mode[i] = mode; e_borrow[i] = borrowing; }
+}
+
 #define KB_FLAT_THREADS 1024
 #ifndef KB_FLAT_NG
 #define KB_FLAT_NG 8  // lanes per entry in the nominate phase
@@ -206,7 +404,7 @@ __global__ void __launch_bounds__(KB_FLAT_THREADS) k_cycle_flat(const __grid_con
   int *n_e = (int *)(smem_raw + Y.n_e), *n_wl = (int *)(smem_raw + Y.n_wl), *n_ps0 = (int *)(smem_raw + Y.n_ps0), *n_psn = (int *)(smem_raw + Y.n_psn);
   int *e_gid = (int *)(smem_raw + Y.e_gid), *e_cq = (int *)(smem_raw + Y.e_cq), *e_prio = (int *)(smem_raw + Y.e_prio), *e_ident = (int *)(smem_raw + Y.e_ident);
   int *e_psn = (int *)(smem_raw + Y.e_psn), *e_wl = (int *)(smem_raw + Y.e_wl), *e_ps0 = (int *)(smem_raw + Y.e_ps0);
-  i64 *e_ts = (i64 *)(smem_raw + Y.e_ts), *e_lg = (i64 *)(smem_raw + Y.e_lg); uint8_t *e_qr = smem_raw + Y.e_qr;
+  i64 *e_ts = (i64 *)(smem_raw + Y.e_ts), *e_lg = (i64 *)(smem_raw + Y.e_lg); uint8_t *e_qr = smem_raw + Y.e_qr, *e_flat = smem_raw + Y.e_flat;
   int *e_mode = (int *)(smem_raw + Y.e_mode), *e_borrow = (int *)(smem_raw + Y.e_borrow), *e_rank = (int *)(smem_raw + Y.e_rank);
   int *s_sorted = (int *)(smem_raw + Y.sorted), *m_sorted = (int *)(smem_raw + Y.m_sorted); uint32_t *ok_bits = (uint32_t *)(smem_raw + Y.d_sorted);
   int *r_gid = (int *)(smem_raw + Y.r_gid), *r_count = (int *)(smem_raw + Y.r_count), *r_min = (int *)(smem_raw + Y.r_min);
@@ -408,9 +606,11 @@ __global__ void __launch_bounds__(KB_FLAT_THREADS) k_cycle_flat(const __grid_con
     const int ps0 = e_ps0[i], l0 = e_psn[i], np = e_psn[i + 1] - l0;
     const int pr = __ldg(D.wl_priority + wl); const i64 ts = __ldg(D.wl_ts + wl), lg = __ldg(D.wl_last_gen + wl);
     const uint8_t qr = D.wl_has_qr ? __ldg(D.wl_has_qr + wl) : 0;
+    bool single = np == 1;
     for (int k = 0; k < np; k++) {
       const int row = ps0 + k, l = l0 + k;
       const int cnt = __ldg(D.ps_count + row), mn = __ldg(D.ps_min_count + row); const uint32_t msk = __ldg(D.ps_req_mask + row);
+      if ((D.flags & KB_F_PARTIAL_ADMISSION) && mn >= 0 && cnt > mn) single = false;  // the PodSetReducer may run
       const int grp = D.ps_group ? __ldg(D.ps_group + row) : -1; const u64 ok = __ldg(D.ps_flavor_ok + row);
       for (int r0 = 0; r0 < R; r0 += 4) {
         i64 q[4]; int8_t lt[4];
@@ -422,6 +622,12 @@ __global__ void __launch_bounds__(KB_FLAT_THREADS) k_cycle_flat(const __grid_con
       r_gid[l] = row; r_count[l] = cnt; r_min[l] = mn; r_mask[l] = msk; r_group[l] = grp; r_ok[l] = ok;
     }
     e_prio[i] = pr; e_ts[i] = ts; e_lg[i] = lg; e_qr[i] = qr;
+    bool covers_pods = false;  // the ClusterQueue has a resource group with the pods resource (assign_workload_coop)
+    if (single && D.pods_res >= 0) {
+      const int32_t *rgs = (const int32_t *)(s_blob + BH->rgs); const uint32_t *rgmask = (const uint32_t *)(s_blob + BH->rgmask);
+      for (int g = rgs[e_cq[i]]; g < rgs[e_cq[i] + 1]; g++) if (rgmask[g] & (1u << D.pods_res)) covers_pods = true;
+    }
+    e_flat[i] = (single ? KB_FLAT_WALK : 0) | (covers_pods ? KB_FLAT_PODS : 0);
   }
   KB_PP(1, 6);
   for (int i = tid; i < tb; i += nthreads) {
@@ -480,10 +686,8 @@ __global__ void __launch_bounds__(KB_FLAT_THREADS) k_cycle_flat(const __grid_con
     for (int i0 = 0; i0 < n; i0 += groups) {
       const int i = i0 + tid / KB_FLAT_NG;
       if (i < n) {  // whole lane groups take the branch together
-        bool need_search = false;
-        int borrowing;
-        const int mode = get_assignments_coop<KB_FLAT_NG>(L, &need_search, i, &borrowing, gmask, gbase, glane);
-        if (glane == 0) { e_mode[i] = mode; e_borrow[i] = borrowing; }
+        if (e_flat[i] & KB_FLAT_WALK) flat_walk<KB_FLAT_NG>(D, Y, smem_raw, i, gmask, gbase, glane);
+        else flat_generic_assign<KB_FLAT_NG>(L, i, gmask, gbase, glane, e_mode, e_borrow);
       }
     }
   }
@@ -501,13 +705,25 @@ __global__ void __launch_bounds__(KB_FLAT_THREADS) k_cycle_flat(const __grid_con
   __syncthreads();
   KB_PP(2, 4);
   {
+    auto share = [&](int i, int r) { return e_flat[i] & KB_FLAT_WALK ? flat_share_ratio(D, Y, smem_raw, i, r) : entry_share_ratio(L, i, r); };
     const int half = nthreads / 2;
     if (tid < half) {
-      if (split) { for (int c = tid; c < n * R; c += half) s_ratio[(size_t)(c / R) * 4 + c % R] = entry_share_ratio(L, c / R, c % R); }  // one division per thread
-      else for (int i = tid; i < n; i += half) compute_entry_key(L, i, s_key + (size_t)i * 4);
+      if (split) { for (int c = tid; c < n * R; c += half) s_ratio[(size_t)(c / R) * 4 + c % R] = share(c / R, c % R); }  // one division per thread
+      else
+        for (int i = tid; i < n; i += half) {
+          double best = 0.0;
+          if (fair) for (int r = 0; r < R; r++) { const double ratio = share(i, r); if (ratio > best) best = ratio; }
+          flat_key_finish(D, Y, smem_raw, i, fair, best, s_key + (size_t)i * 4);
+        }
     } else {
       for (int i = tid - half; i < n; i += half) {
-        expand_entry(L, i, s_q + (size_t)i * FR);
+        if (e_flat[i] & KB_FLAT_WALK) {  // expand_entry: one podset, one cell per assigned resource
+          const int l = e_psn[i];
+          for (int r = 0; r < R; r++) {
+            const int f = o_fl[(size_t)l * R + r];
+            if (f >= 0) s_q[(size_t)i * FR + f * R + r] = (e_flat[i] & KB_FLAT_PODS) && r == D.pods_res ? (i64)o_cnt[l] : r_req[(size_t)l * R + r];
+          }
+        } else expand_entry(L, i, s_q + (size_t)i * FR);
       }
     }
   }
@@ -517,7 +733,7 @@ __global__ void __launch_bounds__(KB_FLAT_THREADS) k_cycle_flat(const __grid_con
     for (int i = tid; i < n; i += nthreads) {
       double best = 0.0;
       for (int r = 0; r < R; r++) { const double ratio = s_ratio[(size_t)i * 4 + r]; if (ratio > best) best = ratio; }
-      entry_key_finish(L, i, true, best, s_key + (size_t)i * 4);  // overwrites the entry's own four slots
+      flat_key_finish(D, Y, smem_raw, i, true, best, s_key + (size_t)i * 4);  // overwrites the entry's own four slots
     }
   }
   KB_PP(2, 6);

@@ -1539,95 +1539,125 @@ extern "C" int32_t kb_tas_find(kb_handle *h, const kb_tas_topology *t, const kb_
   }
   size_t max_slots = 1, max_round = 1;
   for (int rd = 0; rd < n_rounds; rd++) { max_slots = std::max(max_slots, round_slot_req[rd].size()); max_round = std::max(max_round, round_req[rd].size()); }
-  std::vector<int32_t> tmp_start(NQ + 1, 0);
-  for (int q = 0; q < NQ; q++) tmp_start[q + 1] = tmp_start[q] + std::max(0, std::min(r->count[q], NL));
-  const int list_cap = max_count + 8;
+  int max_level = 1;  // no list of a level is longer than the level
+  for (int l = 0; l < L; l++) max_level = std::max(max_level, t->level_start[l + 1] - t->level_start[l]);
+  // Lists and output regions are sized for assignments of at most `count` leaves.  Overcommitted leaves (negative free
+  // capacity, so negative counts: requests.go CountIn) can make an assignment longer; such a request reports the size
+  // it needed and the whole call runs again with larger buffers, which keeps the chains' order.
+  std::vector<int32_t> region(std::max(1, NQ), 0);
+  for (int q = 0; q < NQ; q++) region[q] = std::max(0, std::min(r->count[q], NL));
+  int list_cap = std::min(max_count, max_level) + 8;
   const int sel_grid = (int)std::min<size_t>(max_round, (size_t)h->sm_count * 8);
-  // ---- device buffer (grow-only)
-  size_t tot = 0;
-  auto need = [&](size_t n, size_t sz) { tot += pad256(n * sz); };
-  need(L + 1, 4); need(ND, 4); need(ND + 1, 4); need((size_t)NL * R, 8); need(NL, 4); need((size_t)NL * R, 8); need(NL, 4);
-  need((size_t)NQ * R, 8); for (int k = 0; k < 10; k++) need(NQ, 4); need(r->leaf_ok ? (size_t)NQ * ok_words : 1, 4);
-  need(max_slots * ND, 4); need(max_slots * ND, 4); need((size_t)n_chain_slots * NL * R, 8); need((size_t)n_chain_slots * NL, 4);
-  need(NQ + 1, 4); need(NQ + 1, 4); need(NQ + 2, 4); need(tmp_start[NQ] + 1, 4); need(tmp_start[NQ] + 1, 4);
-  need((size_t)sel_grid * 6 * list_cap, 4); need(max_round, 4); need(max_slots, 4); need(std::max(1, out->capacity), 4); need(std::max(1, out->capacity), 4);
-  if (tot > h->tas_buf_cap) {
-    if (h->tas_buf) cudaFree(h->tas_buf);
-    h->tas_buf = nullptr; h->tas_buf_cap = 0;
-    CUDA_TRY(h, cudaMalloc(&h->tas_buf, tot + (1 << 20)));
-    h->tas_buf_cap = tot + (1 << 20);
-  }
-  size_t used = 0;
-  auto take = [&](size_t n, size_t sz) { char *p = h->tas_buf + used; used += pad256(n * sz); return p; };
-  auto upl = [&](const void *src, size_t n, size_t sz) -> char * { char *d = take(n, sz); if (n) cudaMemcpyAsync(d, src, n * sz, cudaMemcpyHostToDevice, h->stream); return d; };
-  TasDev T{};
-  T.L = L; T.n_domains = ND; T.n_leaves = NL; T.leaf0 = leaf0; T.R = R; T.pods_res = t->pods_resource; T.n_req = NQ;
-  T.level_start = (const int32_t *)upl(t->level_start, L + 1, 4); T.parent = (const int32_t *)upl(t->parent, ND, 4);
-  T.child_start = (const int32_t *)upl(cstart.data(), ND + 1, 4);
-  T.free_cap = (const i64 *)upl(t->free_capacity, (size_t)NL * R, 8); T.cap_mask = (const uint32_t *)upl(t->cap_mask, NL, 4);
-  T.tas_usage = (const i64 *)upl(t->tas_usage, (size_t)NL * R, 8); T.usage_mask = (const uint32_t *)upl(t->usage_mask, NL, 4);
-  T.pod_request = (const i64 *)upl(r->pod_request, (size_t)NQ * R, 8); T.request_mask = (const uint32_t *)upl(r->request_mask, NQ, 4);
-  T.flags = (const uint32_t *)upl(r->flags, NQ, 4); T.count = (const int32_t *)upl(r->count, NQ, 4);
-  T.slice_size = (const int32_t *)upl(r->slice_size, NQ, 4); T.level = (const int32_t *)upl(r->level, NQ, 4);
-  T.slice_level = (const int32_t *)upl(r->slice_level, NQ, 4);
-  T.slot = (const int32_t *)upl(slot.data(), NQ, 4); T.chain_slot = (const int32_t *)upl(chain_slot.data(), NQ, 4); T.pred = (const int32_t *)upl(pred.data(), NQ, 4);
-  T.leaf_ok = r->leaf_ok ? (const uint32_t *)upl(r->leaf_ok, (size_t)NQ * ok_words, 4) : nullptr; T.ok_words = ok_words;
-  T.state = (int32_t *)take(max_slots * ND, 4); T.slice = (int32_t *)take(max_slots * ND, 4);
-  T.assumed = (i64 *)take((size_t)n_chain_slots * NL * R, 8); T.assumed_mask = (uint32_t *)take((size_t)n_chain_slots * NL, 4);
-  if (n_chain_slots) { cudaMemsetAsync(T.assumed, 0, (size_t)n_chain_slots * NL * R * 8, h->stream); cudaMemsetAsync(T.assumed_mask, 0, (size_t)n_chain_slots * NL * 4, h->stream); }
-  T.status = (int32_t *)take(NQ + 1, 4); T.n_out = (int32_t *)take(NQ + 1, 4);
-  int32_t *d_asg_start = (int32_t *)take(NQ + 2, 4);
-  T.tmp_start = (int32_t *)upl(tmp_start.data(), NQ + 1, 4);
-  T.tmp_leaf = (int32_t *)take(tmp_start[NQ] + 1, 4); T.tmp_count = (int32_t *)take(tmp_start[NQ] + 1, 4);
-  T.lists = (int32_t *)take((size_t)sel_grid * 6 * list_cap, 4); T.list_cap = list_cap;
-  int32_t *d_round = (int32_t *)take(max_round, 4), *d_slotreq = (int32_t *)take(max_slots, 4);
-  int32_t *d_leaf = (int32_t *)take(std::max(1, out->capacity), 4), *d_cnt = (int32_t *)take(std::max(1, out->capacity), 4);
-  if (NQ) cudaMemsetAsync(T.n_out, 0, (size_t)(NQ + 1) * 4, h->stream);
-  CUDA_TRY(h, cudaEventRecord(h->ev2, h->stream));
-  h->kev_n = 0;
-  int launches = 0;
-  for (int rd = 0; rd < n_rounds; rd++) {
-    int ns = (int)round_slot_req[rd].size(), nr = (int)round_req[rd].size();
-    CUDA_TRY(h, cudaMemcpyAsync(d_slotreq, round_slot_req[rd].data(), (size_t)ns * 4, cudaMemcpyHostToDevice, h->stream));
-    CUDA_TRY(h, cudaMemcpyAsync(d_round, round_req[rd].data(), (size_t)nr * 4, cudaMemcpyHostToDevice, h->stream));
-    if (rd == 0) kmark(h, KB_K_TAS_LEAF);
-    k_tas_leaf<<<dim3((NL + 255) / 256, ns), 256, 0, h->stream>>>(T, d_slotreq, ns); launches++;
-    if (rd == 0) kmark(h, KB_K_TAS_REDUCE);
-    for (int l = L - 2; l >= 0; l--) {
-      int n = t->level_start[l + 1] - t->level_start[l];
-      k_tas_reduce<<<dim3((n + 127) / 128, ns), 128, 0, h->stream>>>(T, d_slotreq, ns, l); launches++;
+  std::vector<int32_t> grow(NQ + 2, 0);
+  for (;;) {
+    std::vector<int32_t> tmp_start(NQ + 1, 0);
+    for (int q = 0; q < NQ; q++) tmp_start[q + 1] = tmp_start[q] + region[q];
+    // ---- device buffer (grow-only)
+    size_t tot = 0;
+    auto need = [&](size_t n, size_t sz) { tot += pad256(n * sz); };
+    need(L + 1, 4); need(ND, 4); need(ND + 1, 4); need((size_t)NL * R, 8); need(NL, 4); need((size_t)NL * R, 8); need(NL, 4);
+    need((size_t)NQ * R, 8); for (int k = 0; k < 10; k++) need(NQ, 4); need(r->leaf_ok ? (size_t)NQ * ok_words : 1, 4);
+    need(max_slots * ND, 4); need(max_slots * ND, 4); need((size_t)n_chain_slots * NL * R, 8); need((size_t)n_chain_slots * NL, 4);
+    need(NQ + 1, 4); need(NQ + 2, 4); need((size_t)n_rounds * max_slots, 4); need(NQ + 1, 4); need(NQ + 2, 4);
+    need(tmp_start[NQ] + 1, 4); need(tmp_start[NQ] + 1, 4);
+    need((size_t)sel_grid * 6 * list_cap, 4); need(max_round, 4); need(max_slots, 4); need(std::max(1, out->capacity), 4); need(std::max(1, out->capacity), 4);
+    if (tot > h->tas_buf_cap) {
+      if (h->tas_buf) cudaFree(h->tas_buf);
+      h->tas_buf = nullptr; h->tas_buf_cap = 0;
+      CUDA_TRY(h, cudaMalloc(&h->tas_buf, tot + (1 << 20)));
+      h->tas_buf_cap = tot + (1 << 20);
     }
-    if (rd == 0) kmark(h, KB_K_TAS_SELECT);
-    k_tas_select<<<std::min(nr, sel_grid), KB_TAS_THREADS, 0, h->stream>>>(T, d_round, nr); launches++;
-    if (rd == 0) kmark(h, KB_K_TAS);
+    size_t used = 0;
+    auto take = [&](size_t n, size_t sz) { char *p = h->tas_buf + used; used += pad256(n * sz); return p; };
+    auto upl = [&](const void *src, size_t n, size_t sz) -> char * { char *d = take(n, sz); if (n) cudaMemcpyAsync(d, src, n * sz, cudaMemcpyHostToDevice, h->stream); return d; };
+    TasDev T{};
+    T.L = L; T.n_domains = ND; T.n_leaves = NL; T.leaf0 = leaf0; T.R = R; T.pods_res = t->pods_resource; T.n_req = NQ;
+    T.level_start = (const int32_t *)upl(t->level_start, L + 1, 4); T.parent = (const int32_t *)upl(t->parent, ND, 4);
+    T.child_start = (const int32_t *)upl(cstart.data(), ND + 1, 4);
+    T.free_cap = (const i64 *)upl(t->free_capacity, (size_t)NL * R, 8); T.cap_mask = (const uint32_t *)upl(t->cap_mask, NL, 4);
+    T.tas_usage = (const i64 *)upl(t->tas_usage, (size_t)NL * R, 8); T.usage_mask = (const uint32_t *)upl(t->usage_mask, NL, 4);
+    T.pod_request = (const i64 *)upl(r->pod_request, (size_t)NQ * R, 8); T.request_mask = (const uint32_t *)upl(r->request_mask, NQ, 4);
+    T.flags = (const uint32_t *)upl(r->flags, NQ, 4); T.count = (const int32_t *)upl(r->count, NQ, 4);
+    T.slice_size = (const int32_t *)upl(r->slice_size, NQ, 4); T.level = (const int32_t *)upl(r->level, NQ, 4);
+    T.slice_level = (const int32_t *)upl(r->slice_level, NQ, 4);
+    T.slot = (const int32_t *)upl(slot.data(), NQ, 4); T.chain_slot = (const int32_t *)upl(chain_slot.data(), NQ, 4); T.pred = (const int32_t *)upl(pred.data(), NQ, 4);
+    T.leaf_ok = r->leaf_ok ? (const uint32_t *)upl(r->leaf_ok, (size_t)NQ * ok_words, 4) : nullptr; T.ok_words = ok_words;
+    T.state = (int32_t *)take(max_slots * ND, 4); T.slice = (int32_t *)take(max_slots * ND, 4);
+    T.assumed = (i64 *)take((size_t)n_chain_slots * NL * R, 8); T.assumed_mask = (uint32_t *)take((size_t)n_chain_slots * NL, 4);
+    if (n_chain_slots) { cudaMemsetAsync(T.assumed, 0, (size_t)n_chain_slots * NL * R * 8, h->stream); cudaMemsetAsync(T.assumed_mask, 0, (size_t)n_chain_slots * NL * 4, h->stream); }
+    // zeroed together: n_out, grow, the negative-leaf flags of every round's slots
+    T.n_out = (int32_t *)take(NQ + 1, 4); T.grow = (int32_t *)take(NQ + 2, 4);
+    int32_t *d_neg = (int32_t *)take((size_t)n_rounds * max_slots, 4);
+    CUDA_TRY(h, cudaMemsetAsync(T.n_out, 0, (char *)h->tas_buf + used - (char *)T.n_out, h->stream));
+    T.status = (int32_t *)take(NQ + 1, 4);
+    int32_t *d_asg_start = (int32_t *)take(NQ + 2, 4);
+    T.tmp_start = (int32_t *)upl(tmp_start.data(), NQ + 1, 4);
+    T.tmp_leaf = (int32_t *)take(tmp_start[NQ] + 1, 4); T.tmp_count = (int32_t *)take(tmp_start[NQ] + 1, 4);
+    T.lists = (int32_t *)take((size_t)sel_grid * 6 * list_cap, 4); T.list_cap = list_cap;
+    int32_t *d_round = (int32_t *)take(max_round, 4), *d_slotreq = (int32_t *)take(max_slots, 4);
+    int32_t *d_leaf = (int32_t *)take(std::max(1, out->capacity), 4), *d_cnt = (int32_t *)take(std::max(1, out->capacity), 4);
+    CUDA_TRY(h, cudaEventRecord(h->ev2, h->stream));
+    h->kev_n = 0;
+    int launches = 0;
+    for (int rd = 0; rd < n_rounds; rd++) {
+      int ns = (int)round_slot_req[rd].size(), nr = (int)round_req[rd].size();
+      CUDA_TRY(h, cudaMemcpyAsync(d_slotreq, round_slot_req[rd].data(), (size_t)ns * 4, cudaMemcpyHostToDevice, h->stream));
+      CUDA_TRY(h, cudaMemcpyAsync(d_round, round_req[rd].data(), (size_t)nr * 4, cudaMemcpyHostToDevice, h->stream));
+      T.neg = d_neg + (size_t)rd * max_slots;
+      if (rd == 0) kmark(h, KB_K_TAS_LEAF);
+      k_tas_leaf<<<dim3((NL + 255) / 256, ns), 256, 0, h->stream>>>(T, d_slotreq, ns); launches++;
+      if (rd == 0) kmark(h, KB_K_TAS_REDUCE);
+      for (int l = L - 2; l >= 0; l--) {
+        int n = t->level_start[l + 1] - t->level_start[l];
+        k_tas_reduce<<<dim3((n + 127) / 128, ns), 128, 0, h->stream>>>(T, d_slotreq, ns, l); launches++;
+      }
+      if (rd == 0) kmark(h, KB_K_TAS_SELECT);
+      k_tas_select<<<std::min(nr, sel_grid), KB_TAS_THREADS, 0, h->stream>>>(T, d_round, nr); launches++;
+      if (rd == 0) kmark(h, KB_K_TAS);
+    }
+    if (NQ) {
+      k_scan_i32<<<1, 1024, 0, h->stream>>>(T.n_out, d_asg_start, NQ); launches++;
+      k_tas_compact<<<NQ, 64, 0, h->stream>>>(T, d_asg_start, d_leaf, d_cnt, out->capacity); launches++;
+    }
+    kmark(h, -1);
+    CUDA_TRY(h, cudaEventRecord(h->ev3, h->stream));
+    CUDA_TRY(h, cudaGetLastError());
+    if (NQ) {
+      CUDA_TRY(h, cudaMemcpyAsync(out->status, T.status, (size_t)NQ * 4, cudaMemcpyDeviceToHost, h->stream));
+      CUDA_TRY(h, cudaMemcpyAsync(out->asg_start, d_asg_start, (size_t)(NQ + 1) * 4, cudaMemcpyDeviceToHost, h->stream));
+      CUDA_TRY(h, cudaMemcpyAsync(grow.data(), T.grow, 2 * 4, cudaMemcpyDeviceToHost, h->stream));
+    } else out->asg_start[0] = 0;
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    if (grow[0] || grow[1]) {  // some request overflowed its list or its output region: enlarge them and run again
+      bool larger = false;
+      if (grow[0] > list_cap) {
+        if (grow[0] > max_level) return fail(h, KB_ERR_INVALID, "tas: a list is longer than its level");
+        list_cap = std::min(max_level, std::max(grow[0], 2 * list_cap));
+        larger = true;
+      }
+      if (grow[1]) {
+        CUDA_TRY(h, cudaMemcpy(grow.data() + 2, T.grow + 2, (size_t)NQ * 4, cudaMemcpyDeviceToHost));
+        for (int q = 0; q < NQ; q++) if (grow[2 + q] > region[q]) { region[q] = grow[2 + q]; larger = true; }
+      }
+      if (!larger) return fail(h, KB_ERR_INVALID, "tas: overflow without a larger buffer to retry with");
+      continue;
+    }
+    out->n_assigned = out->asg_start[NQ];
+    int ncopy = std::min(out->n_assigned, out->capacity);
+    if (ncopy > 0) {
+      CUDA_TRY(h, cudaMemcpy(out->asg_leaf, d_leaf, (size_t)ncopy * 4, cudaMemcpyDeviceToHost));
+      CUDA_TRY(h, cudaMemcpy(out->asg_count, d_cnt, (size_t)ncopy * 4, cudaMemcpyDeviceToHost));
+    }
+    { float ms = 0; cudaEventElapsedTime(&ms, h->ev2, h->ev3); h->stats.last_cycle_gpu_ms = ms; }
+    h->stats.kernel_launches = launches;
+    for (int i = 0; i < KB_N_KERNELS; i++) h->stats.kernel_ms[i] = 0.f;
+    for (int i = 0; i + 1 < h->kev_n; i++) {
+      float kms = 0; cudaEventElapsedTime(&kms, h->kev[i], h->kev[i + 1]);
+      if (h->kev_id[i] >= 0) h->stats.kernel_ms[h->kev_id[i]] += kms;
+    }
+    if (out->n_assigned > out->capacity) return fail(h, KB_ERR_CAPACITY, "tas: assignment buffer too small");
+    return KB_OK;
   }
-  if (NQ) {
-    k_scan_i32<<<1, 1024, 0, h->stream>>>(T.n_out, d_asg_start, NQ); launches++;
-    k_tas_compact<<<NQ, 64, 0, h->stream>>>(T, d_asg_start, d_leaf, d_cnt, out->capacity); launches++;
-  }
-  kmark(h, -1);
-  CUDA_TRY(h, cudaEventRecord(h->ev3, h->stream));
-  CUDA_TRY(h, cudaGetLastError());
-  if (NQ) {
-    CUDA_TRY(h, cudaMemcpyAsync(out->status, T.status, (size_t)NQ * 4, cudaMemcpyDeviceToHost, h->stream));
-    CUDA_TRY(h, cudaMemcpyAsync(out->asg_start, d_asg_start, (size_t)(NQ + 1) * 4, cudaMemcpyDeviceToHost, h->stream));
-  } else out->asg_start[0] = 0;
-  CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-  out->n_assigned = out->asg_start[NQ];
-  int ncopy = std::min(out->n_assigned, out->capacity);
-  if (ncopy > 0) {
-    CUDA_TRY(h, cudaMemcpy(out->asg_leaf, d_leaf, (size_t)ncopy * 4, cudaMemcpyDeviceToHost));
-    CUDA_TRY(h, cudaMemcpy(out->asg_count, d_cnt, (size_t)ncopy * 4, cudaMemcpyDeviceToHost));
-  }
-  { float ms = 0; cudaEventElapsedTime(&ms, h->ev2, h->ev3); h->stats.last_cycle_gpu_ms = ms; }
-  h->stats.kernel_launches = launches;
-  for (int i = 0; i < KB_N_KERNELS; i++) h->stats.kernel_ms[i] = 0.f;
-  for (int i = 0; i + 1 < h->kev_n; i++) {
-    float kms = 0; cudaEventElapsedTime(&kms, h->kev[i], h->kev[i + 1]);
-    if (h->kev_id[i] >= 0) h->stats.kernel_ms[h->kev_id[i]] += kms;
-  }
-  if (out->n_assigned > out->capacity) return fail(h, KB_ERR_CAPACITY, "tas: assignment buffer too small");
-  return KB_OK;
 }
 
 extern "C" int32_t kb_tree_eval(kb_handle *h, const kb_snapshot *s, kb_tree_out *out) {

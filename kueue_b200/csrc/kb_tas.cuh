@@ -33,7 +33,15 @@ struct TasDev {
   int32_t *status, *n_out, *tmp_start, *tmp_leaf, *tmp_count;
   // per-CTA lists of k_tas_select
   int32_t *lists; int list_cap;
+  // grow[0]: longest list a request needed beyond list_cap; grow[1]: requests whose output region was too small;
+  // grow[2 + q]: entries request q needed.  A request that overflows stores nothing and reports KB_TAS_GROW; the host
+  // reruns the whole call with larger buffers.
+  int32_t *grow;
+  // per shape slot of the current round: some leaf has a negative count (overcommitted: free capacity below zero)
+  int32_t *neg;
 };
+// internal status of a request that needs larger buffers (never returned: kb_tas_find reruns)
+#define KB_TAS_GROW 3
 
 // slot descriptors: which request defines the shape of slot s (its request row / mask / flags / eligibility / chain)
 __global__ void k_tas_leaf(TasDev T, const int32_t *slot_req, int n_slots) {
@@ -63,6 +71,7 @@ __global__ void k_tas_leaf(TasDev T, const int32_t *slot_req, int n_slots) {
       if (!have || c < result) { result = c; have = true; }
     }
     st = have ? result : 0;
+    if (st < 0) T.neg[s] = 1;
   }
   const int L = T.L;
   T.state[(size_t)s * T.n_domains + T.leaf0 + lf] = st;
@@ -124,8 +133,9 @@ struct TasSel {
   bool lfc;                // LeastFreeCapacity order (:1291-1294)
   TasKey *s_red;
   TasKey *s_cache; int *s_cmeta;  // sorted candidate cache of a large level set + {a, b, filter, arg, n valid, complete}
-  // sort key of sortedDomains :1495-1515: sliceState (desc, or asc under LeastFreeCapacity), state asc, levelValues asc
-  __device__ __forceinline__ TasKey key(int d) const { TasKey k; k.v = 0; k.k0 = lfc ? sl[d] : -sl[d]; k.k1 = st[d]; k.d = d; return k; }
+  // sort key of sortedDomains :1495-1515: sliceState (desc, or asc under LeastFreeCapacity), state asc, levelValues asc.
+  // ~x = -x - 1 reverses the order of every int32, INT32_MIN included (a truncated CountIn can produce it)
+  __device__ __forceinline__ TasKey key(int d) const { TasKey k; k.v = 0; k.k0 = lfc ? sl[d] : ~sl[d]; k.k1 = st[d]; k.d = d; return k; }
   template <typename F> __device__ inline void for_each(const TasSet &S, F f) const {
     if (!S.parents) { for (int d = S.a + threadIdx.x; d < S.b; d += blockDim.x) f(d); return; }
     for (int i = 0; i < S.np; i++) {
@@ -135,8 +145,9 @@ struct TasSel {
   }
   // next domain of S in sorted order strictly after `after` (after.d < 0: the first).  filter 1: only domains whose
   // sliceState >= arg; filter 2 / 3: skip domains whose sliceState / state is 0 — the reference appends them with zero
-  // pods (they sort first under LeastFreeCapacity), which changes nothing downstream: their descendants get zero
-  // pods and buildTopologyAssignmentForLevels drops zero counts (:1443-1446)
+  // pods (they sort first under LeastFreeCapacity), which changes nothing downstream while no count is negative: their
+  // descendants get zero pods and buildTopologyAssignmentForLevels drops zero counts (:1443-1446).  A zero domain
+  // over a negative leaf does hand pods to its descendants, so a shape with a negative leaf walks with filter 0.
   // Large level sets (tens of thousands of hosts) are walked through a sorted CACHE of their smallest keys: one pass
   // keeps every thread's KB_TAS_LOCAL best candidates, the block sorts their union in shared memory, and all keys up
   // to T = the smallest "worst kept key" among the threads that had to drop something are provably complete (every
@@ -254,6 +265,8 @@ __device__ inline void tas_select_one(const TasDev &T, const int q, TasKey *s_re
   const int levelIdx = T.level[q], sliceLevel = T.slice_level[q], L = T.L;
   const bool required = flags & KB_TAS_REQUIRED, unconstrained = flags & KB_TAS_UNCONSTRAINED;
   auto finish = [&](int status, int n) { if (threadIdx.x == 0) { T.status[q] = status; T.n_out[q] = n; } };
+  // a list longer than list_cap: record its length and give up (kb_tas_find reruns with larger lists)
+  auto grow_lists = [&](int n) { if (threadIdx.x == 0) atomicMax(&T.grow[0], n); finish(KB_TAS_GROW, 0); };
   if (T.pred[q] >= 0 && T.status[T.pred[q]] != KB_TAS_OK) { finish(-1, 0); return; }  // the chain stopped at an earlier podset (:551-553)
   if (levelIdx < 0 || levelIdx >= L || sliceLevel < 0 || sliceLevel >= L || levelIdx > sliceLevel || sliceSize < 1) { finish(KB_TAS_BAD_REQUEST, 0); return; }
   const int slot = T.slot[q];
@@ -261,6 +274,8 @@ __device__ inline void tas_select_one(const TasDev &T, const int q, TasKey *s_re
   if (threadIdx.x == 0) s_cmeta[4] = -1;  // the cache belongs to one request (its shape's counts)
   __syncthreads();
   const bool lfc = X.lfc;
+  const bool skip0 = !T.neg[slot];
+  const int f_slices = skip0 ? 2 : 0, f_pods = skip0 ? 3 : 0;
   const TasKey none{0, 0, 0, -1};
   // ---- findLevelWithFitDomains :1200-1282 (no leaders)
   int ncur = 0, fitLevel = levelIdx;
@@ -282,7 +297,7 @@ __device__ inline void tas_select_one(const TasDev &T, const int q, TasKey *s_re
       TasKey cur = none;
       ncur = 0;
       while (remaining > 0) {
-        TasKey d = X.next(S, cur, 2, 0);
+        TasKey d = X.next(S, cur, f_slices, 0);
         if (d.d < 0) break;
         cur = d;
         if (!lfc && X.sl[d.d] >= remaining) d = X.best_fit(S, d, remaining, true);
@@ -290,7 +305,8 @@ __device__ inline void tas_select_one(const TasDev &T, const int q, TasKey *s_re
         ncur++;
         remaining -= X.sl[d.d];
       }
-      if (remaining > 0 || ncur > cap) { finish(KB_TAS_NO_FIT, 0); return; }
+      if (remaining > 0) { finish(KB_TAS_NO_FIT, 0); return; }
+      if (ncur > cap) { grow_lists(ncur); return; }
       fitLevel = lv;
       break;
     }
@@ -322,23 +338,24 @@ __device__ inline void tas_select_one(const TasDev &T, const int q, TasKey *s_re
     ncur = s_n;
     int32_t *t; t = c_d; c_d = n_d; n_d = t; t = c_st; c_st = n_st; n_st = t; t = c_sl; c_sl = n_sl; n_sl = t;
   }
-  // ordered greedy over a SET (children of parents) walked in sorted order; appends to the next-level list
+  // ordered greedy over a SET (children of parents) walked in sorted order; appends to the next-level list.  Entries
+  // past list_cap are counted, not stored: the walk itself reads only the current list.
   auto update_set = [&](const TasSet &S, int32_t cnt, int32_t ss, bool slices, int *nn) -> bool {
     int32_t remaining = slices ? cnt / ss : cnt;
     TasKey cur = none;
     while (true) {
-      TasKey d = X.next(S, cur, remaining > 0 ? (slices ? 2 : 3) : 0, 0);
+      TasKey d = X.next(S, cur, remaining > 0 ? (slices ? f_slices : f_pods) : 0, 0);
       if (d.d < 0) return false;
       cur = d;
       int32_t v = slices ? X.sl[d.d] : X.st[d.d];
       if (!lfc && v >= remaining) { d = X.best_fit(S, d, remaining, slices); v = slices ? X.sl[d.d] : X.st[d.d]; }
-      if (*nn >= cap) return false;
+      const bool store = threadIdx.x == 0 && *nn < cap;
       if (v >= remaining) {
-        if (threadIdx.x == 0) { n_d[*nn] = d.d; n_st[*nn] = slices ? remaining * ss : remaining; n_sl[*nn] = slices ? remaining : X.sl[d.d]; }
+        if (store) { n_d[*nn] = d.d; n_st[*nn] = slices ? remaining * ss : remaining; n_sl[*nn] = slices ? remaining : X.sl[d.d]; }
         (*nn)++;
         return true;
       }
-      if (threadIdx.x == 0) { n_d[*nn] = d.d; n_st[*nn] = slices ? v * ss : v; n_sl[*nn] = X.sl[d.d]; }
+      if (store) { n_d[*nn] = d.d; n_st[*nn] = slices ? v * ss : v; n_sl[*nn] = X.sl[d.d]; }
       (*nn)++;
       remaining -= v;
     }
@@ -349,6 +366,7 @@ __device__ inline void tas_select_one(const TasDev &T, const int q, TasKey *s_re
     TasSet S{0, 0, c_d, ncur};
     int nn = 0;
     if (!update_set(S, count, sliceSize, true, &nn)) { finish(KB_TAS_NO_FIT, 0); return; }
+    if (nn > cap) { grow_lists(nn); return; }
     __syncthreads();
     ncur = nn;
     int32_t *t; t = c_d; c_d = n_d; n_d = t; t = c_st; c_st = n_st; n_st = t; t = c_sl; c_sl = n_sl; n_sl = t;
@@ -360,21 +378,29 @@ __device__ inline void tas_select_one(const TasDev &T, const int q, TasKey *s_re
       TasSet S{0, 0, c_d + i, 1};
       if (!update_set(S, c_st[i], 1, false, &nn)) { finish(KB_TAS_NO_FIT, 0); return; }
     }
+    if (nn > cap) { grow_lists(nn); return; }
     __syncthreads();
     ncur = nn;
     int32_t *t; t = c_d; c_d = n_d; n_d = t; t = c_st; c_st = n_st; n_st = t; t = c_sl; c_sl = n_sl; n_sl = t;
   }
   __syncthreads();
-  // ---- buildAssignment :1455-1466: leaves in lexicographic (= index) order, zero counts dropped
+  // ---- buildAssignment :1455-1466: leaves in lexicographic (= index) order, zero counts dropped.  Negative counts
+  // (overcommitted leaves) can make the assignment longer than the podset's count, hence than its output region.
+  if (threadIdx.x == 0) { int n = 0; for (int j = 0; j < ncur; j++) if (c_st[j] != 0) n++; s_n = n; }
+  __syncthreads();
+  const int nout = s_n;
   const int out0 = T.tmp_start[q];
-  int nout = 0;
+  if (nout > T.tmp_start[q + 1] - out0) {
+    if (threadIdx.x == 0) { T.grow[2 + q] = nout; atomicAdd(&T.grow[1], 1); }
+    finish(KB_TAS_GROW, 0);
+    return;
+  }
   for (int i = threadIdx.x; i < ncur; i += blockDim.x) {
     if (c_st[i] == 0) continue;
     int rank = 0;
     for (int j = 0; j < ncur; j++) if (c_st[j] != 0 && c_d[j] < c_d[i]) rank++;
     T.tmp_leaf[out0 + rank] = c_d[i] - T.leaf0; T.tmp_count[out0 + rank] = c_st[i];
   }
-  if (threadIdx.x == 0) { for (int j = 0; j < ncur; j++) if (c_st[j] != 0) nout++; }
   // ---- addAssumedUsage :619-627 for the next podset of the chain
   const int cs = T.chain_slot[q];
   if (cs >= 0) {
